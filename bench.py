@@ -22,6 +22,12 @@ One STEP = one complete solve of the workload (b = A*1, x0 = 0, to BICG_TOL / MA
                 sample = the first REF_ITERS iterations of the same solve
 
 --impl reference times that CPU build alone (rank 0 only under torchrun); it never loads the product library.
+
+--dump-outputs DIR writes what the last timed solve returned to its caller, so that two builds can be compared output
+for output (the inputs depend only on the arguments): x.npy and r.npy (the solution and the recursive residual),
+history.npy (dot_r/dot_zero per iteration) and iterations.npy, all float64.  Under torchrun every rank writes its own
+row block with a _rank<R> suffix.  Where x and r would exceed 64 MB in all, a fixed seeded sample of rows is written
+instead, with their global row numbers in index.npy.
 """
 import argparse
 import json
@@ -51,6 +57,7 @@ WORKLOADS = {
 }
 BYTES_PER_ITER_N = {"bicgstab": 160, "ca_bicgstab": 216, "pipe_bicgstab": 232}   # SURVEY.md 8(d)
 REF_ITERS = 100        # iterations per reference step: ~1-2 s of CPU work per step, init SpMV amortised over 100
+DUMP_BYTES = 60 << 20  # --dump-outputs: x and r of all ranks together stay below this (history and index come on top)
 
 
 def measured_peak():
@@ -423,6 +430,9 @@ def run_b200(args, w):
         final_res, converged = st.final_res, st.converged
         hist = B.last_history().copy()          # full-precision residual history of the last resident solve (parity object)
         last_iters = int(st.iters)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"x": x_dev.cpu().numpy(), "r": r_dev.cpu().numpy(), "history": hist,
+                                             "iterations": np.array([last_iters])}, rank, world, int(blk.displs[rank]))
 
         # roofline of the dominant kernel, measured live (per rank; rank 0 reported)
         peak, peak_src = measured_peak()
@@ -565,6 +575,19 @@ def run_b200(args, w):
         print(json.dumps(line))
 
 
+def dump_outputs(d, outputs, rank, world, row0):
+    """One float64 .npy per output of the rank's last timed solve; x and r shrink to the same seeded rows on every run
+    when all ranks' x and r together exceed DUMP_BYTES."""
+    os.makedirs(d, exist_ok=True)
+    n = outputs["x"].size
+    if world * 2 * 8 * n > DUMP_BYTES:
+        idx = np.sort(np.random.default_rng(rank).choice(n, size=DUMP_BYTES // (world * 3 * 8), replace=False))
+        outputs = dict(outputs, x=outputs["x"][idx], r=outputs["r"][idx], index=row0 + idx)
+    suffix = f"_rank{rank}" if world > 1 else ""
+    for name, a in outputs.items():
+        np.save(os.path.join(d, f"{name}{suffix}.npy"), np.asarray(a, dtype=np.float64))
+
+
 def read_traffic(key):
     """dram bytes measured by ncu (committed under profiles/spmv_traffic.json), else None."""
     try:
@@ -583,7 +606,10 @@ def main():
     ap.add_argument("--workload", default="transport", choices=sorted(WORKLOADS))
     ap.add_argument("--method", default=None)
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed solve's outputs to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of --impl b200")
     w = dict(WORKLOADS[args.workload])
     if args.method:
         w["method"] = args.method

@@ -37,6 +37,24 @@ def global_csr(B, kind, g, p0, seed=12345):
     return blk, blk.n, ptr, col, val
 
 
+def sha256(a):
+    """Digest of a float64 vector's bytes: golden files store it in place of vectors too large to keep whole."""
+    import hashlib
+    return hashlib.sha256(np.ascontiguousarray(a, dtype="<f8").tobytes()).hexdigest()
+
+
+def write_mtx(path, n, ptr, col, val):
+    """Matrix-Market file of a CSR matrix, column-major like SuiteSparse files, with a comment and a blank line."""
+    import scipy.sparse as sp
+    A = sp.csr_matrix((val, col, ptr), shape=(n, n)).tocsc().tocoo()
+    with open(path, "w") as fh:
+        fh.write("%%MatrixMarket matrix coordinate real general\n% comment\n\n")
+        fh.write(f"{n} {n} {A.nnz}\n")
+        for r, c, v in zip(A.row, A.col, A.data):
+            fh.write(f"{r + 1} {c + 1} {float(v)!r}\n")
+    return A
+
+
 def rel_err(a, b):
     a, b = np.asarray(a, dtype=np.float64), np.asarray(b, dtype=np.float64)
     return np.abs(a - b).max() / max(np.abs(b).max(), 1e-300)
@@ -49,7 +67,7 @@ def big_csr(kind, g, p0, tmpdir="/dev/shm"):
     """Full-size synthetic matrix as (file, n, ptr, col, val): written once per session by the stand-alone generator
     oracle/gen_csr (binary layout of oracle.py: write_csr_bin), so neither numpy index gymnastics nor a second copy of the
     1.6 M-row matrix is needed.  The file is what oracle/_ref/ref_driver_* reads."""
-    import os, subprocess, tempfile
+    import atexit, os, shutil, subprocess, tempfile
     key = (kind, g, p0)
     if key not in _BIG:
         root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -57,6 +75,7 @@ def big_csr(kind, g, p0, tmpdir="/dev/shm"):
         if not os.path.exists(gen):
             subprocess.run(["make", "-C", os.path.join(root, "oracle"), "oracle"], check=True)
         d = tempfile.mkdtemp(dir=tmpdir if os.path.isdir(tmpdir) else None)
+        atexit.register(shutil.rmtree, d, True)           # a few hundred MB of shared memory per matrix
         f = os.path.join(d, f"{kind}_{g}.bin")
         kinds = {"stencil15": 0, "laplace5": 1, "random": 2, "convdiff": 3}
         subprocess.run([gen, str(kinds[kind]), str(int(g)), repr(float(p0)), f], check=True, capture_output=True)

@@ -87,33 +87,33 @@ def test_generators_match_block_split_of_global(B):
             assert a.diag.cols == a.n_loc and a.offd.cols == g1.n                 # matrix.c:344, 351
 
 
+def _checks():
+    return np.load(os.path.join(ROOT, "tests", "golden", "ref_checks.npz"))
+
+
 def test_matrix_market_loader(B, O, tmp_path):
-    """MPI_csr_load_matrix_block: same blocks as the reference's loader (checked via the compiled reference when
-    present, else via the generator the file was written from); in-row order = file order (stable row sort)."""
+    """MPI_csr_load_matrix_block: same blocks as the generator the file was written from; in-row order = file order
+    (stable row sort).  The reference program itself (main.c unchanged) solves the same file in as many iterations as the
+    oracle: its count is golden, and the program is run too where oracle/_ref is built."""
+    from helpers import write_mtx
     blk = B.gen_block("convdiff", 12, 1.5)
     n = blk.n
     ptr, col, val = B.block_to_global_csr(blk)
-    import scipy.sparse as sp
-    A = sp.csr_matrix((val, col, ptr), shape=(n, n)).tocsc().tocoo()          # column-major like SuiteSparse files
     f = tmp_path / "a.mtx"
-    with open(f, "w") as fh:
-        fh.write("%%MatrixMarket matrix coordinate real general\n% comment\n\n")
-        fh.write(f"{n} {n} {A.nnz}\n")
-        for r, c, v in zip(A.row, A.col, A.data):
-            fh.write(f"{r + 1} {c + 1} {float(v)!r}\n")
+    A = write_mtx(f, n, ptr, col, val)
     got = B.load_matrix_block(f, world=1)
     assert (got.n, got.n_loc, int(got.info.nz)) == (n, n, A.nnz) and got.info.code == b"MCRG"
     for u, v in zip(got.diag_arrays(), blk.diag_arrays()):
         assert np.array_equal(np.asarray(u), np.asarray(v))
     assert got.offd.nz == 0 and got.offd.rows == n and got.offd.cols == n
+    b = O.spmv(n, ptr, col, val, np.ones(n))
+    it = O.solve("bicgstab", n, ptr, col, val, b, tol=1e-10, max_iter=500)["iters"]
+    assert it == int(_checks()["mm_cd12|iters"])
     ref_main = os.path.join(ROOT, "oracle", "_ref", "ref_main_hist")
     if os.path.exists(ref_main):
-        # the reference program itself (main.c unchanged) on the same file: same iteration count as the oracle
         env = dict(os.environ, REF_EPS="1e-10", REF_MAX_ITER="500", REF_OUT_ITER="1", MALLOC_MMAP_THRESHOLD_="0")
         out = subprocess.run([ref_main, str(f), "bicgstab"], env=env, capture_output=True, text=True, check=True).stdout
-        it_ref = int(re.search(r"Total iter\s*:\s*(\d+)", out).group(1))
-        b = O.spmv(n, ptr, col, val, np.ones(n))
-        assert O.solve("bicgstab", n, ptr, col, val, b, tol=1e-10, max_iter=500)["iters"] == it_ref
+        assert it == int(re.search(r"Total iter\s*:\s*(\d+)", out).group(1))
 
 
 def test_matrix_market_pattern_and_errors(B, tmp_path):
@@ -141,19 +141,27 @@ def test_compute_entry_points_fail_loudly_without_gpu(B):
     assert p.returncode == 1 and "RETURNED" not in p.stdout and "no usable CUDA device" in p.stderr
 
 
-def test_reference_main_c_links_against_the_library(B, tmp_path):
+def _reference_driver(name):
+    """oracle/_ref/<name>: one of the reference's drivers, UNCHANGED, compiled against include/compat/mpi.h and linked against
+    libbicgstab_b200.so by `make -C oracle ref` (which needs the reference's sources at build time)."""
+    exe = os.path.join(ROOT, "oracle", "_ref", name)
+    if not os.path.exists(exe):
+        pytest.skip(f"oracle/_ref/{name} not built (the reference's sources were absent at build time)")
+    ldd = subprocess.run(["ldd", "-r", exe], capture_output=True, text=True)      # binds every symbol against today's library
+    out = ldd.stdout + ldd.stderr
+    assert ldd.returncode == 0 and "undefined symbol" not in out, out
+    lib = re.search(r"libbicgstab_b200\.so => (\S+)", out)
+    assert lib and os.path.realpath(lib.group(1)) == os.path.realpath(os.path.join(ROOT, "mpi-bicgstab_b200", "libbicgstab_b200.so")), out
+    return exe
+
+
+def test_reference_main_c_links_against_the_library(B):
     """The drop-in claim itself: the reference's main.c, UNCHANGED, compiles against include/compat/mpi.h and
-    links against libbicgstab_b200.so (needs /root/reference, so only in the build container)."""
-    src = "/root/reference/src/main.c"
-    if not os.path.exists(src):
-        pytest.skip("/root/reference not present")
-    exe = tmp_path / "solver"
-    cmd = ["gcc", "-O2", "-w", "-I" + os.path.join(ROOT, "include", "compat"), "-I/root/reference/src", src,
-           "-L" + os.path.dirname(B.LIB_PATH), "-lbicgstab_b200", "-Wl,-rpath," + os.path.dirname(B.LIB_PATH), "-o", str(exe)]
-    subprocess.run(cmd, check=True)
-    p = subprocess.run([str(exe)], capture_output=True, text=True)         # no arguments -> usage text (main.c:64-75)
+    links against libbicgstab_b200.so."""
+    exe = _reference_driver("ref_main_b200")
+    p = subprocess.run([exe], capture_output=True, text=True)              # no arguments -> usage text (main.c:64-75)
     assert "Usage:" in p.stdout and "pipe_bicgstab_rr" in p.stdout
-    undefined = subprocess.run(["nm", "-u", str(exe)], capture_output=True, text=True).stdout
+    undefined = subprocess.run(["nm", "-u", exe], capture_output=True, text=True).stdout
     for sym in ("bicgstab", "ca_bicgstab", "pipe_bicgstab", "pipe_bicgstab_rr", "MPI_csr_spmv_ovlap",
                 "MPI_csr_load_matrix_block", "csr_init_matrix", "csr_free_matrix"):
         assert re.search(r"\bU %s\b" % sym, undefined), sym
@@ -161,17 +169,11 @@ def test_reference_main_c_links_against_the_library(B, tmp_path):
 
 @pytest.mark.parametrize("driver,solver", [("main_shifted.c", "shifted_lopbicg_switching"), ("main_repeat.c", "shifted_lopbicg_switching"),
                                            ("main_seed_diff.c", "shifted_lopbicg_switching")])
-def test_reference_shifted_drivers_link_against_the_library(B, tmp_path, driver, solver):
+def test_reference_shifted_drivers_link_against_the_library(B, driver, solver):
     """The shifted drivers (what the reference's top-level Makefile builds), UNCHANGED: besides the loader / SpMV / solver
     entry points they call vector.h's my_daxpy / my_dcopy on host arrays (main_shifted.c:114-135), which the library exports."""
-    src = "/root/reference/src/" + driver
-    if not os.path.exists(src):
-        pytest.skip("/root/reference not present")
-    exe = tmp_path / "shifted"
-    cmd = ["gcc", "-O2", "-w", "-I" + os.path.join(ROOT, "include", "compat"), "-I/root/reference/src", src,
-           "-L" + os.path.dirname(B.LIB_PATH), "-lbicgstab_b200", "-Wl,-rpath," + os.path.dirname(B.LIB_PATH), "-lm", "-o", str(exe)]
-    subprocess.run(cmd, check=True)
-    undefined = subprocess.run(["nm", "-u", str(exe)], capture_output=True, text=True).stdout
+    exe = _reference_driver("ref_%s_b200" % driver[len("main_"):-len(".c")])
+    undefined = subprocess.run(["nm", "-u", exe], capture_output=True, text=True).stdout
     for sym in (solver, "MPI_csr_spmv_ovlap", "MPI_csr_load_matrix_block", "csr_init_matrix", "my_daxpy"):
         assert re.search(r"\bU %s\b" % sym, undefined), sym
 
@@ -179,19 +181,13 @@ def test_reference_shifted_drivers_link_against_the_library(B, tmp_path, driver,
 def test_unchanged_shifted_driver_reaches_the_library_and_fails_loudly_without_a_gpu(B, tmp_path):
     """main_shifted.c built against the library, run on a small Matrix-Market file: the loader (host code) works, the first
     device call (MPI_csr_spmv_ovlap, main_shifted.c:113) must refuse to run without a GPU -- message + exit(1), no CPU path."""
-    src = "/root/reference/src/main_shifted.c"
-    if not os.path.exists(src):
-        pytest.skip("/root/reference not present")
     import torch
     if torch.cuda.is_available():
         pytest.skip("a GPU is visible: the driver would really run (covered by the -m gpu tests of its library calls)")
-    exe = tmp_path / "shifted"
-    subprocess.run(["gcc", "-O2", "-w", "-I" + os.path.join(ROOT, "include", "compat"), "-I/root/reference/src", src,
-                    "-L" + os.path.dirname(B.LIB_PATH), "-lbicgstab_b200", "-Wl,-rpath," + os.path.dirname(B.LIB_PATH), "-lm",
-                    "-o", str(exe)], check=True)
+    exe = _reference_driver("ref_shifted_b200")
     mtx = tmp_path / "a.mtx"
     mtx.write_text("%%MatrixMarket matrix coordinate real general\n3 3 5\n1 1 4.0\n2 2 4.0\n3 3 4.0\n1 2 -1.0\n3 2 -1.0\n")
-    p = subprocess.run([str(exe), str(mtx)], capture_output=True, text=True)
+    p = subprocess.run([exe, str(mtx)], capture_output=True, text=True)
     assert p.returncode == 1 and "IO time" in p.stdout and "no usable CUDA device" in p.stderr
 
 
@@ -215,8 +211,8 @@ def test_host_blas1_entry_points_match_the_oracle_bitwise(B, O):
 
 def test_csr_shift_diagonal_matches_the_reference(B, O):
     """matrix.h's csr_shift_diagonal (matrix.c:536-551) on host arrays: same values as the reference's own compiled function
-    (when oracle/_ref is there) and as the definition, a missing diagonal is fatal, and the cached device copy keyed by the
-    arrays is forgotten (no GPU needed: nothing is cached here)."""
+    (its golden output, and the function itself when oracle/_ref is there) and as the definition, a missing diagonal is fatal,
+    and the cached device copy keyed by the arrays is forgotten (no GPU needed: nothing is cached here)."""
     blk = B.gen_block("convdiff", 12, 1.5)
     n = blk.n
     before = np.array(blk.diag_arrays()[0][:int(blk.diag.nz)], dtype=np.float64)
@@ -225,6 +221,7 @@ def test_csr_shift_diagonal_matches_the_reference(B, O):
     want = before.copy()
     rows = np.repeat(np.arange(n), np.diff(ptr))
     want[col == rows] += 0.37
+    assert np.array_equal(_checks()["shiftdiag_cd12|val"], want)
     if O.have_ref("libref_strict.so"):
         import ctypes
         L = O.ref_lib("strict")

@@ -39,11 +39,12 @@ def test_reference_main_c_two_ranks(tmp_path):
     sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "oracle")); sys.path.insert(0, os.path.join(ROOT, "tests"))
     import mpi_bicgstab_b200 as B
     import oracle as O
-    from test_gpu_parity import _write_mtx
+    from helpers import write_mtx
     blk = B.gen_block("stencil15", 12, 14.0)
     f = tmp_path / "s12.mtx"
-    ptr, col, val = _write_mtx(f, blk, B)
     n = blk.n
+    ptr, col, val = B.block_to_global_csr(blk)
+    write_mtx(f, n, ptr, col, val)
     env = dict(os.environ, BICG_TOL="1e-10", BICG_MAX_ITER="600")
     p = subprocess.run([os.path.join(ROOT, "tools", "bicgrun"), "-np", "2", exe, str(f), "bicgstab"],
                        capture_output=True, text=True, env=env, timeout=300)
