@@ -184,12 +184,15 @@ int bicg_profile_solve(bicg_matrix *m, int method, int iters, double class_ms[3]
  *   bicg_debug_get_vec / _get_scalars: arena vector `id` / {rTr rTr_old rTs rTy yTy rTw wTw rTz dot_r dot_zero alpha
  *                         beta omega} as the last solve on this handle left them.
  *   bicg_debug_resident_ctas: how many CTAs of the last persistent-kernel launch on this handle kept their matrix slice in
- *                         shared memory for the whole solve (BICG_RESIDENT, csrc/mega.cu). */
+ *                         shared memory for the whole solve (BICG_RESIDENT, csrc/mega.cu).
+ *   bicg_debug_mega_tiles: the number of tiles of the persistent-kernel plan (0: no usable plan); *narrow = how many of them
+ *                         stream their columns as 16-bit tile-relative codes instead of 32-bit indices (csrc/mega.cu). */
 int bicg_debug_vec_phase(bicg_matrix *m, int phase, const double coef[3], double *vecs, double dots[8]);
 int bicg_debug_spmv_epi(bicg_matrix *m, int epi, double *vecs, double dots[8]);
 int bicg_debug_get_vec(bicg_matrix *m, int id, double *out);
 int bicg_debug_get_scalars(bicg_matrix *m, double out[13]);
 int bicg_debug_resident_ctas(bicg_matrix *m);
+int bicg_debug_mega_tiles(bicg_matrix *m, int *narrow);
 
 /* full-precision history of the last solve on this rank: out[k] = dot_r/dot_zero after iteration k
  * (out[0] = 1).  Returns the number of entries available (iters + 1). */

@@ -73,6 +73,7 @@ SYMBOLS = {
     "bicg_debug_get_vec": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p]),
     "bicg_debug_get_scalars": (C.c_int, [C.c_void_p, _P(C.c_double)]),
     "bicg_debug_resident_ctas": (C.c_int, [C.c_void_p]),
+    "bicg_debug_mega_tiles": (C.c_int, [C.c_void_p, _P(C.c_int)]),
     "bicg_last_history": (C.c_int, [_P(C.c_double), C.c_int]),
     "bicg_last_stats": (_P(bicg_stats), []),
     "bicg_stream": (C.c_void_p, []),

@@ -291,6 +291,12 @@ class DeviceMatrix:
         """CTAs of the last persistent-kernel launch that kept their matrix slice in shared memory (BICG_RESIDENT)."""
         return int(lib.bicg_debug_resident_ctas(self.h))
 
+    def mega_tiles(self):
+        """(tiles, narrow): tiles of the persistent-kernel plan and how many of them stream 16-bit column codes."""
+        narrow = C.c_int()
+        tiles = lib.bicg_debug_mega_tiles(self.h, C.byref(narrow))
+        return int(tiles), int(narrow.value)
+
     def spmv_time(self, reps=20):
         ms, by = C.c_double(), C.c_double()
         lib.bicg_spmv_time(self.h, reps, C.byref(ms), C.byref(by))

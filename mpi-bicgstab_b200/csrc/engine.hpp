@@ -152,6 +152,9 @@ struct MegaPlan {
     int *d_cta_tile = nullptr;
     int4 *d_cta_dep = nullptr;
     int *d_tile_flag = nullptr;  // only when rows longer than a stage were cut into chunk tiles
+    int narrow = 0;              // tiles whose columns are streamed as 16-bit codes (mega.cu: StageHdr::cbase)
+    int *d_tile_cbase = nullptr; // only when narrow > 0: per tile the column base, -1 for a wide tile
+    unsigned short *d_col16 = nullptr;   // only when narrow > 0: nnz + 16 codes, those of the narrow tiles filled in
     bool chunked = false;
     std::vector<int> cta_row;    // grid + 1: first row of every CTA
 };

@@ -524,10 +524,27 @@ static void build_mega_plan(bicg_matrix *m, const unsigned *h_ptr, const std::ve
         BICG_CUDA(cudaMemcpy(mp.d_cta_tile, cta_tile.data(), cta_tile.size() * sizeof(int), cudaMemcpyHostToDevice));
         launch_mega_dep(m->d_col, m->d_ptr, mp.d_tile_row, mp.d_cta_tile, G, m->ghost_off, mp.d_cta_dep, c.stream);   // behind the upload
         BICG_CUDA(cudaGetLastError());
+        // the column width of every tile, from the merged columns on the device; the 16-bit copy of the columns only exists
+        // when some tile can use it.  Its padding (like d_col's) covers the 8-entry windows the kernel copies.
+        int *d_cbase = (int *)c.dev_alloc(((size_t)mp.ntiles + 1) * sizeof(int));
+        BICG_CUDA(cudaMemsetAsync(d_cbase + mp.ntiles, 0, sizeof(int), c.stream));
+        launch_mega_tile_base(m->d_col, mp.d_tile_nz, mp.d_tile_flag, mp.ntiles, m->ghost_off, d_cbase, d_cbase + mp.ntiles, c.stream);
+        BICG_CUDA(cudaGetLastError());
+        BICG_CUDA(cudaMemcpyAsync(&mp.narrow, d_cbase + mp.ntiles, sizeof(int), cudaMemcpyDeviceToHost, c.stream));
+        BICG_CUDA(cudaStreamSynchronize(c.stream));
+        if (mp.narrow > 0) {
+            mp.d_tile_cbase = d_cbase;
+            mp.d_col16 = (unsigned short *)c.dev_alloc((m->nnz + 16) * sizeof(unsigned short));
+            BICG_CUDA(cudaMemsetAsync(mp.d_col16, 0, (m->nnz + 16) * sizeof(unsigned short), c.stream));
+            launch_mega_tile_codes(m->d_col, mp.d_tile_nz, mp.d_tile_cbase, mp.ntiles, mp.d_col16, c.stream);
+            BICG_CUDA(cudaGetLastError());
+        } else {
+            c.dev_free(d_cbase);
+        }
         mp.ok = true;
         if (c.cfg.verbose)
-            fprintf(stderr, "[bicg mega r%d] threads=%d lanes=%d stages=%d cap=%d tiles=%d smem=%zu resident_smem=%zu\n", m->rank, threads, lanes,
-                    stages, cap, mp.ntiles, mp.smem, mp.res_smem);
+            fprintf(stderr, "[bicg mega r%d] threads=%d lanes=%d stages=%d cap=%d tiles=%d narrow=%d smem=%zu resident_smem=%zu\n", m->rank,
+                    threads, lanes, stages, cap, mp.ntiles, mp.narrow, mp.smem, mp.res_smem);
         return;
     }
 }
@@ -863,7 +880,7 @@ void matrix_destroy(bicg_matrix *m)
     free_plan(m->plan);
     c.dev_free(m->d_trace);
     c.dev_free(m->mega.d_tile_row); c.dev_free(m->mega.d_tile_nz); c.dev_free(m->mega.d_cta_tile); c.dev_free(m->mega.d_cta_dep);
-    c.dev_free(m->mega.d_tile_flag);
+    c.dev_free(m->mega.d_tile_flag); c.dev_free(m->mega.d_tile_cbase); c.dev_free(m->mega.d_col16);
     if (m->hist_extra) cudaFree(m->hist_extra);
     c.dev_free(m->d_val); c.dev_free(m->d_col); c.dev_free(m->d_ptr);
     if (m->world > 1) c.arena_pool.emplace(m->arena_bytes, Context::ArenaRec{m->arena, m->arena_bytes, m->arena_id, m->arena_handle});

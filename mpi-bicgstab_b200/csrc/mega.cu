@@ -42,7 +42,9 @@ namespace {
 constexpr int PROW_PAD = 8;
 constexpr int RED_THREADS = MEGA_MAX_CTAS;          // one polled slot per thread
 constexpr int RED_WARPS = RED_THREADS / 32;
-struct StageHdr { int row0, row1; unsigned a0; int rowa; unsigned lo, hi; int flag; int pad_; };   // lo, hi: the tile's entries relative to a0
+// lo, hi: the tile's entries relative to a0.  cbase >= 0: a narrow tile -- the column region of the stage holds 16-bit codes
+// col - cbase from entry (a0 & ~7) on (TMA wants 16-byte windows), so entry a0 + i has its code at index i + (a0 & 4)
+struct StageHdr { int row0, row1; unsigned a0; int rowa; unsigned lo, hi; int flag; int cbase; };
 
 __device__ __forceinline__ void mbar_arrive(unsigned bar)
 {
@@ -525,48 +527,61 @@ struct Mega {
                 if (lane == 0) mbar_arrive(smem_u32(&sh.empty_bar[s]));
                 continue;
             }
-            const int row = h.row0 + row_in_tile;
-            const bool valid = row < h.row1;
-            int j = 0, e = 0;
-            double e0 = 0.0, e1 = 0.0, e2 = 0.0, e3 = 0.0;     // epilogue operands: in flight during the gathers
-            if (valid) {
-                j = (int)(sptr[row - h.rowa] - h.a0) + sub;
-                e = (int)(sptr[row - h.rowa + 1] - h.a0);
-                if (sub == 0) {
-                    if (EPI == EPI_RH_Y) e0 = a.v.rh[row];
-                    if (EPI == EPI_QY_YY) e0 = a.v.r[row];
-                    if (EPI == EPI_CA4) { e0 = a.v.rh[row]; e1 = a.v.r[row]; e2 = a.v.s[row]; e3 = a.v.z[row]; }
-                }
-            }
-            double acc = 0.0;
-            while (j < e) {
-                unsigned c[UNR];
-                double v[UNR], xv[UNR];
-#pragma unroll
-                for (int u = 0; u < UNR; ++u) {
-                    const int idx = min(j + u * LANES, e - 1);
-                    c[u] = scol[idx];
-                    v[u] = sval[idx];
-                }
-#pragma unroll
-                for (int u = 0; u < UNR; ++u) xv[u] = CG ? ld_l2(x + c[u]) : ld_coherent(x + c[u]);
-#pragma unroll
-                for (int u = 0; u < UNR; ++u)
-                    if (j + u * LANES < e) acc = fma(v[u], xv[u], acc);
-                j += UNR * LANES;
-            }
-            acc = lanes_sum<LANES>(acc);
-            if (valid && sub == 0) {
-                y[row] = acc;
-                if (EPI == EPI_RH_Y) dot[0] = fma(e0, acc, dot[0]);
-                if (EPI == EPI_QY_YY) { dot[0] = fma(e0, acc, dot[0]); dot[1] = fma(acc, acc, dot[1]); }
-                if (EPI == EPI_CA4) {
-                    dot[0] = fma(e0, e1, dot[0]); dot[1] = fma(e0, acc, dot[1]);
-                    dot[2] = fma(e0, e2, dot[2]); dot[3] = fma(e0, e3, dot[3]);
-                }
-            }
+            // the branch is uniform over the CTA (one header per stage)
+            if (h.cbase >= 0)
+                tile_rows<EPI, CG>(h, sval, reinterpret_cast<const unsigned short *>(scol) + (h.a0 & 4u), sptr, x + h.cbase, y,
+                                   dot, sub, row_in_tile);
+            else
+                tile_rows<EPI, CG>(h, sval, scol, sptr, x, y, dot, sub, row_in_tile);
             __syncwarp();
             if (lane == 0) mbar_arrive(smem_u32(&sh.empty_bar[s]));
+        }
+    }
+    // one tile of whole rows: LANES threads per row, a row's entries accumulated in storage order.  ColT = unsigned short (narrow
+    // tile): scol holds the codes col - cbase and xb = x + cbase; ColT = unsigned: scol holds the columns and xb = x.
+    template <int EPI, bool CG, typename ColT>
+    __device__ __forceinline__ void tile_rows(const StageHdr &h, const double *sval, const ColT *scol, const unsigned *sptr,
+                                              const double *xb, double *y, double (&dot)[4], int sub, int row_in_tile)
+    {
+        const int row = h.row0 + row_in_tile;
+        const bool valid = row < h.row1;
+        int j = 0, e = 0;
+        double e0 = 0.0, e1 = 0.0, e2 = 0.0, e3 = 0.0;     // epilogue operands: in flight during the gathers
+        if (valid) {
+            j = (int)(sptr[row - h.rowa] - h.a0) + sub;
+            e = (int)(sptr[row - h.rowa + 1] - h.a0);
+            if (sub == 0) {
+                if (EPI == EPI_RH_Y) e0 = a.v.rh[row];
+                if (EPI == EPI_QY_YY) e0 = a.v.r[row];
+                if (EPI == EPI_CA4) { e0 = a.v.rh[row]; e1 = a.v.r[row]; e2 = a.v.s[row]; e3 = a.v.z[row]; }
+            }
+        }
+        double acc = 0.0;
+        while (j < e) {
+            unsigned c[UNR];
+            double v[UNR], xv[UNR];
+#pragma unroll
+            for (int u = 0; u < UNR; ++u) {
+                const int idx = min(j + u * LANES, e - 1);
+                c[u] = scol[idx];
+                v[u] = sval[idx];
+            }
+#pragma unroll
+            for (int u = 0; u < UNR; ++u) xv[u] = CG ? ld_l2(xb + c[u]) : ld_coherent(xb + c[u]);
+#pragma unroll
+            for (int u = 0; u < UNR; ++u)
+                if (j + u * LANES < e) acc = fma(v[u], xv[u], acc);
+            j += UNR * LANES;
+        }
+        acc = lanes_sum<LANES>(acc);
+        if (valid && sub == 0) {
+            y[row] = acc;
+            if (EPI == EPI_RH_Y) dot[0] = fma(e0, acc, dot[0]);
+            if (EPI == EPI_QY_YY) { dot[0] = fma(e0, acc, dot[0]); dot[1] = fma(acc, acc, dot[1]); }
+            if (EPI == EPI_CA4) {
+                dot[0] = fma(e0, e1, dot[0]); dot[1] = fma(e0, acc, dot[1]);
+                dot[2] = fma(e0, e2, dot[2]); dot[3] = fma(e0, e3, dot[3]);
+            }
         }
     }
 
@@ -902,20 +917,26 @@ __global__ void __launch_bounds__(CT + 32, 1) bicg_mega_kernel(const __grid_cons
                 const unsigned p0 = a.tile_nz[t], p1 = a.tile_nz[t + 1];
                 const unsigned a0 = p0 & ~3u, cnt = ((p1 + 3u) & ~3u) - a0;
                 const int rowa = row0 & ~3, cntp = ((row1 + 1 + 3) & ~3) - rowa;
+                // narrow tile: codes from entry p0 & ~7 to p1 rounded up to 8 -- at most 2 (tile entries + 14) bytes, which
+                // the 4 cap bytes of the column region always hold (cap >= tile entries + 8).  A narrow tile has entries.
+                const int cbase = a.tile_cbase ? a.tile_cbase[t] : -1;
+                const unsigned c0 = p0 & ~7u;
+                const void *csrc = cbase >= 0 ? (const void *)(a.col16 + c0) : (const void *)(a.col + a0);
+                const unsigned cbytes = cbase >= 0 ? (((p1 + 7u) & ~7u) - c0) * 2u : cnt * 4u;
                 unsigned char *st = dyn_smem + (size_t)s * stage_bytes;
                 double   *sval = reinterpret_cast<double *>(st);
                 unsigned *scol = reinterpret_cast<unsigned *>(sval + cap);
                 unsigned *sptr = scol + cap;
-                sh.hdr[s] = StageHdr{row0, row1, a0, rowa, p0 - a0, p1 - a0, a.tile_flag ? a.tile_flag[t] : 0, 0};
+                sh.hdr[s] = StageHdr{row0, row1, a0, rowa, p0 - a0, p1 - a0, a.tile_flag ? a.tile_flag[t] : 0, cbase};
                 const unsigned bar = smem_u32(&sh.full_bar[s]);
-                mbar_arrive_expect_tx(bar, cnt * 12u + (unsigned)cntp * 4u);
+                mbar_arrive_expect_tx(bar, cnt * 8u + cbytes + (unsigned)cntp * 4u);
                 if (cnt) {
                     if (hint) {
                         tma_load_1d_hint(smem_u32(sval), a.val + a0, cnt * 8u, bar, pol);
-                        tma_load_1d_hint(smem_u32(scol), a.col + a0, cnt * 4u, bar, pol);
+                        tma_load_1d_hint(smem_u32(scol), csrc, cbytes, bar, pol);
                     } else {
                         tma_load_1d(smem_u32(sval), a.val + a0, cnt * 8u, bar);
-                        tma_load_1d(smem_u32(scol), a.col + a0, cnt * 4u, bar);
+                        tma_load_1d(smem_u32(scol), csrc, cbytes, bar);
                     }
                 }
                 tma_load_1d(smem_u32(sptr), a.ptr + rowa, (unsigned)cntp * 4u, bar);
@@ -1033,6 +1054,39 @@ __global__ void __launch_bounds__(256) mega_dep_kernel(const unsigned *__restric
     if (threadIdx.x == 0) dep[blockIdx.x] = make_int4(s[0], s[1], s[2], s[3]);
 }
 
+// one CTA per tile: column base of a narrow tile, -1 for a wide one (see launch_mega_tile_base)
+__global__ void __launch_bounds__(256) mega_tile_base_kernel(const unsigned *__restrict__ col, const unsigned *__restrict__ tile_nz,
+                                                             const int *__restrict__ tile_flag, int ghost_off, int *tile_cbase,
+                                                             int *narrow_count)
+{
+    __shared__ int s[2];
+    if (threadIdx.x == 0) { s[0] = 0x7fffffff; s[1] = -1; }
+    __syncthreads();
+    const int t = blockIdx.x;
+    const unsigned p0 = tile_nz[t], p1 = tile_nz[t + 1];
+    int lo = 0x7fffffff, hi = -1;
+    for (unsigned j = p0 + threadIdx.x; j < p1; j += blockDim.x) {
+        const int c = (int)col[j];
+        lo = min(lo, c); hi = max(hi, c);
+    }
+    atomicMin(&s[0], lo); atomicMax(&s[1], hi);
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        const bool narrow = (tile_flag == nullptr || tile_flag[t] == 0) && p1 > p0 && s[1] < ghost_off && s[1] - s[0] < 65536;
+        tile_cbase[t] = narrow ? s[0] : -1;
+        if (narrow) atomicAdd(narrow_count, 1);
+    }
+}
+
+__global__ void __launch_bounds__(256) mega_tile_codes_kernel(const unsigned *__restrict__ col, const unsigned *__restrict__ tile_nz,
+                                                              const int *__restrict__ tile_cbase, unsigned short *__restrict__ col16)
+{
+    const int t = blockIdx.x;
+    const int base = tile_cbase[t];
+    if (base < 0) return;
+    for (unsigned j = tile_nz[t] + threadIdx.x; j < tile_nz[t + 1]; j += blockDim.x) col16[j] = (unsigned short)((int)col[j] - base);
+}
+
 template <int CT, int LANES>
 cudaError_t launch(const MegaArgs &a, int grid, size_t smem, cudaStream_t st)
 {
@@ -1090,6 +1144,18 @@ void launch_mega_dep(const unsigned *col, const unsigned *ptr, const int *tile_r
                      int ghost_off, int4 *dep, cudaStream_t st)
 {
     mega_dep_kernel<<<grid, 256, 0, st>>>(col, ptr, tile_row, cta_tile, ghost_off, dep);
+}
+
+void launch_mega_tile_base(const unsigned *col, const unsigned *tile_nz, const int *tile_flag, int ntiles, int ghost_off,
+                           int *tile_cbase, int *narrow_count, cudaStream_t st)
+{
+    mega_tile_base_kernel<<<ntiles, 256, 0, st>>>(col, tile_nz, tile_flag, ghost_off, tile_cbase, narrow_count);
+}
+
+void launch_mega_tile_codes(const unsigned *col, const unsigned *tile_nz, const int *tile_cbase, int ntiles,
+                            unsigned short *col16, cudaStream_t st)
+{
+    mega_tile_codes_kernel<<<ntiles, 256, 0, st>>>(col, tile_nz, tile_cbase, col16);
 }
 
 } // namespace bicg

@@ -60,6 +60,9 @@ struct MegaArgs {
     const unsigned *tile_nz;    // ntiles + 1
     const int      *cta_tile;   // grid + 1 : first tile of every CTA (contiguous ownership)
     const int      *tile_flag;  // null, or per tile: 0 whole rows, 1 / 2 chunk of ONE long row (more follow / last)
+    const int      *tile_cbase; // null, or per tile: >= 0 a narrow tile, its columns are streamed as col16 = col - tile_cbase;
+                                //    -1 a wide tile (32-bit col).  Null: every tile is wide
+    const unsigned short *col16;
     int cap, stages;
     int ghost_off;
     int l2_hint;                // 1: matrix stream is loaded with an L2 evict-first policy
@@ -93,5 +96,12 @@ __host__ __device__ inline size_t mega_resident_bytes(unsigned nnz, int rows)
 // per-CTA column ranges of the plan (one launch at plan time)
 void   launch_mega_dep(const unsigned *col, const unsigned *ptr, const int *tile_row, const int *cta_tile, int grid,
                        int ghost_off, int4 *dep, cudaStream_t st);
+// Column width of every tile of the plan (one CTA per tile).  A tile is narrow when it holds whole rows, has entries, none of
+// them in the ghost window, and max col - min col < 65536: tile_cbase[t] = min col, else -1.  narrow_count += narrow tiles.
+void   launch_mega_tile_base(const unsigned *col, const unsigned *tile_nz, const int *tile_flag, int ntiles, int ghost_off,
+                             int *tile_cbase, int *narrow_count, cudaStream_t st);
+// col16[j] = col[j] - tile_cbase[t] for the entries of the narrow tiles
+void   launch_mega_tile_codes(const unsigned *col, const unsigned *tile_nz, const int *tile_cbase, int ntiles,
+                              unsigned short *col16, cudaStream_t st);
 
 } // namespace bicg

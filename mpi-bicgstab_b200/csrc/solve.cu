@@ -91,6 +91,7 @@ struct Seq {
         a.val = m->d_val; a.col = m->d_col; a.ptr = m->d_ptr;
         a.tile_row = m->mega.d_tile_row; a.tile_nz = m->mega.d_tile_nz; a.cta_tile = m->mega.d_cta_tile;
         a.tile_flag = m->mega.d_tile_flag;
+        a.tile_cbase = m->mega.d_tile_cbase; a.col16 = m->mega.d_col16;
         a.cap = m->mega.cap; a.stages = m->mega.stages;
         a.ghost_off = m->ghost_off; a.l2_hint = c.cfg.l2_hint;
         a.gather_cg = c.cfg.gather_cg >= 0 ? c.cfg.gather_cg : 0;
@@ -614,6 +615,12 @@ extern "C" int bicg_debug_resident_ctas(bicg_matrix *m)
     BICG_CUDA(cudaMemcpyAsync(&n, &m->d_msync->st.resident_ctas, sizeof(int), cudaMemcpyDeviceToHost, c.stream));
     BICG_CUDA(cudaStreamSynchronize(c.stream));
     return n;
+}
+
+extern "C" int bicg_debug_mega_tiles(bicg_matrix *m, int *narrow)
+{
+    if (narrow) *narrow = m->mega.ok ? m->mega.narrow : 0;
+    return m->mega.ok ? m->mega.ntiles : 0;
 }
 
 // ------------------------------------------------------------------------------------------------
